@@ -28,6 +28,8 @@ The working set of the sparse layout is ~80 MB: it is L2-resident on purpose, no
           the headline, the exhaustive engine (BIGCLAM_F_LS_EXHAUSTIVE) on the same steps and a whole SGDFindC run from
           the synthetic F0 to the reference's stop rule
 `--impl reference` times that CPU restatement alone (the reference needs a JVM + Spark: absent).
+`--dump-outputs DIR` writes what the timed steps computed (dump_outputs), so that two builds can be compared on the same
+inputs: the graph and F0 are seeded, identical from run to run for the same arguments.
 """
 import argparse
 import ctypes as C
@@ -42,6 +44,7 @@ import numpy as np
 
 REPO = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REPO)
+sys.dont_write_bytecode = True            # the benchmark leaves the tree it runs from as it found it
 
 CONFIGS = {
     "enron50": dict(graph="email-enron", k=50, note="BASELINE config 2 (Email-Enron, reciprocal lines deduplicated)"),
@@ -248,7 +251,7 @@ def measure_traffic(args, kernel_regex):
     cmd = ["ncu", "--metrics", "dram__bytes_read.sum,dram__bytes_write.sum", "--clock-control", "none", "-k", f"regex:{kernel_regex}",
            "--launch-skip", "4", "--launch-count", "1", "--csv", sys.executable, os.path.join(REPO, "tools", "profile_step.py"),
            str(args.k), "5", "2", args.graph]
-    env = dict(os.environ, BIGCLAM_AB_SPARSE="1" if args.layout == "sparse" else "0")
+    env = dict(os.environ, BIGCLAM_AB_SPARSE="1" if args.layout == "sparse" else "0", PYTHONDONTWRITEBYTECODE="1")
     try:
         out = subprocess.run(cmd, capture_output=True, text=True, timeout=180, env=env).stdout
     except Exception as exc:                # noqa: BLE001
@@ -279,6 +282,27 @@ def sparse_layout_bytes(indptr, rp, col):
     cnt = np.diff(indptr)
     blk = 8 * ((cnt + 1) // 2 * 2) + 2 * ((cnt + 7) // 8 * 8)
     return int(blk[col].sum() + 12 * len(col) + 2 * blk.sum() + 16 * (len(rp) - 1))
+
+
+DUMP_F_BYTES = 32 << 20                      # F.npy; with llh.npy and sumF.npy the dump stays below 64 MB
+
+
+def dump_outputs(out_dir, b, llh):
+    """Writes what the hot path hands its caller after the last timed step, as float64 .npy files: llh (the LLH of that
+    step), sumF (K) and F.  F is n x K; when that exceeds DUMP_F_BYTES, the rows of a fixed sample (seed 0, ascending
+    node ids) stand for it, the same rows in every run of the same workload.  Returns a description for the JSON line."""
+    import scipy.sparse as sps
+    indptr, indices, values = b.F_csr()
+    n, k = len(indptr) - 1, b.K
+    m = min(n, DUMP_F_BYTES // (8 * k))
+    rows = np.arange(n) if m == n else np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+    F = sps.csr_matrix((values, indices, indptr), shape=(n, k))[rows].toarray()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "llh.npy"), np.array([llh], dtype=np.float64))
+    np.save(os.path.join(out_dir, "sumF.npy"), b.sumF)
+    np.save(os.path.join(out_dir, "F.npy"), F)
+    return {"dir": out_dir, "files": ["llh.npy", "sumF.npy", "F.npy"],
+            "F_rows": "all" if m == n else f"{m} of {n} rows, np.random.default_rng(0).choice(n, {m}, replace=False), sorted"}
 
 
 class ExtrasWatchdog:
@@ -361,6 +385,7 @@ def run_single(args):
     llh_end = float(b.last_trace[-1])
     tiles = b.tile_stats() if sparse else None
     ls = b.ls_stats() if sparse else None
+    dumped = dump_outputs(args.dump_outputs, b, llh_end) if args.dump_outputs else None    # before e2e moves F on
 
     # ---- roofline of the dominant kernel ----
     peak, peak_src = hbm_peak()
@@ -399,7 +424,7 @@ def run_single(args):
         "l2": ("sparse rows: working set ~2 x %.0f MB, L2-resident by design, no flush" % (layout_bytes / 4e6)) if sparse
               else "inputs (F, 2 buffers) larger than L2, no flush",
         "llh_end": llh_end, "parity": "PARITY UNPINNED: checked against oracle/ (CPU restatement), not against outputs of the reference",
-        "clocks": clocks, "e2e": e2e, "gpu_launches": int(n_all),
+        "clocks": clocks, "e2e": e2e, "gpu_launches": int(n_all), "dumped_outputs": dumped,
         "roofline": {"bound": "hbm", "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak,
                      "traffic": None, "traffic_source": "not reached", "kernel": kernel,
                      "kernel_ms": kavg_ms, "alg_bytes_per_launch": balg, "peak_source": peak_src,
@@ -537,7 +562,13 @@ def main():
     ap.add_argument("--no-line-search", action="store_true", help="skip the exhaustive-line-search arm and the run to convergence")
     ap.add_argument("--extras-limit", type=float, default=420.0,
                     help="seconds the explanatory legs after the timed regions may take before the line is printed without them")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what they computed (llh, sumF, F or a fixed sample of its rows) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.gpus > 1 or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs is implemented for the single-GPU arm (--impl b200 --gpus 1)")
     cfg = CONFIGS[args.config]
     args.graph = args.graph or cfg["graph"]
     args.k = args.k or cfg["k"]

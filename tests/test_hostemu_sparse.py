@@ -10,6 +10,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -112,3 +113,24 @@ def test_bench_prints_its_line_when_an_explanatory_leg_stalls():
     d = _bench_dryrun("--extras-limit", "2")
     assert "extras_cut" in d and d["value"] > 0 and d["e2e"]["value"] > 0 and d["roofline"]["frac"] > 0
     assert d["line_search"] is None or d["line_search"]["run_to_convergence"] is None
+
+
+@pytest.mark.timeout(900)
+def test_bench_dumps_the_state_after_its_timed_steps(oracle, tmp_path):
+    """--dump-outputs: the LLH, sumF and F the hot path returned after the last of the --steps timed steps, i.e. the
+    oracle's state after the warm-up, settle and timed steps from the same seeded workload."""
+    import bench
+    out = str(tmp_path / "dump")
+    d = _bench_dryrun("--steps", "3", "--no-cpu", "--no-init-a", "--no-line-search", "--dump-outputs", out)
+    assert d["steps"] == 3 and d["dumped_outputs"]["F_rows"] == "all"
+    assert sorted(os.listdir(out)) == ["F.npy", "llh.npy", "sumF.npy"]
+    rp, col, F = bench.load_workload("rmat:150:500", 16)
+    s, P = oracle.colsum(F), oracle.make_params(16)
+    for _ in range(d["untimed_steps_before_timing"] + d["steps"]):
+        r = oracle.step(rp, col, F, s, P)
+        F, s = r.F, r.sumF
+    llh, sumF, Fd = (np.load(os.path.join(out, f)) for f in ("llh.npy", "sumF.npy", "F.npy"))
+    assert llh.dtype == sumF.dtype == Fd.dtype == np.float64 and Fd.shape == F.shape
+    assert llh[0] == d["llh_end"] and abs(llh[0] - r.llh) <= 1e-10 * abs(r.llh)
+    assert np.allclose(sumF, s, rtol=1e-11, atol=1e-9)
+    assert np.abs(Fd - F).max() <= 1e-9 * np.abs(F).max()
