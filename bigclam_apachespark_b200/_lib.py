@@ -75,6 +75,8 @@ SIGNATURES = {
     "bigclam_get_kernel_time": (C.c_int, [_vp, _pd, _pi64, _pi64]),
     "bigclam_get_tile_stats": (C.c_int, [_vp, _pi64, _pi64, _pi64, _pi64, _pi64]),
     "bigclam_get_ls_stats": (C.c_int, [_vp, _pi64, _pi64]),
+    "bigclam_set_holdout": (C.c_int, [_vp, _vp, _vp, _vp]),
+    "bigclam_holdout_loglikelihood": (C.c_int, [_vp, _pd, _pi64]),
     "bigclam_retile": (C.c_int, [_vp]),
     "bigclam_set_stream": (C.c_int, [_vp, _vp]),
     "bigclam_device_state": (C.c_int, [_vp, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), _pi64]),

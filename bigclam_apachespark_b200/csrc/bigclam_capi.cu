@@ -14,6 +14,7 @@
 #include <cstdlib>
 #include <numeric>
 #include <string>
+#include <utility>
 #include <vector>
 
 using namespace bigclam;
@@ -119,6 +120,14 @@ struct bigclam_ctx {
     std::vector<int64_t> h_rowptr;                // host copy of the CSR row pointers (order / tile rebuilds)
     std::vector<int32_t> h_col;
     std::vector<int32_t> h_owned;                 // owned nodes (processing order is derived from it)
+    // held-out pairs (bigclam_set_holdout): while set, the steps and the LLH use the masked objective and every node
+    // goes through the general path (tile_step_kernel<.., .., true>: no tiles, no split hubs, no bounds)
+    bool ho = false;
+    int64_t *d_ho_rowptr = nullptr;
+    int32_t *d_ho_col = nullptr;
+    uint8_t *d_ho_edge = nullptr;
+    double *d_ho_part = nullptr;                  // per-node partials of the held-out LLH (n) | their sum
+    int64_t ho_pairs = 0;                         // unordered held-out pairs
 
     std::string err;
 };
@@ -218,6 +227,7 @@ static void free_ctx(bigclam_ctx *c) {
     cudaFree(c->d_pool_top); cudaFree(c->d_overflow);
     cudaFree(c->d_node_llh); cudaFree(c->d_dcnt); cudaFree(c->d_block_part); cudaFree(c->d_ticket);
     cudaFree(c->d_tiles); cudaFree(c->d_tcol); cudaFree(c->d_stats);
+    cudaFree(c->d_ho_rowptr); cudaFree(c->d_ho_col); cudaFree(c->d_ho_edge); cudaFree(c->d_ho_part);
     if (c->x_ipc)
         for (int r = 0; r < c->x_world; ++r)
             if (r != c->x_rank) {
@@ -283,7 +293,7 @@ static int rebuild_sparse_lists(bigclam_ctx *ctx, const std::vector<NodeMeta> &m
     // of edges (a 1,383-edge node of Email-Enron walked by one warp WAS the launch: 1.3 ms for 367 K entries)
     // (BIGCLAM_SPARSE_HUB_DEG overrides the threshold: tests)
     int32_t nh = 0;
-    if (ctx->nsteps <= 16) {
+    if (ctx->nsteps <= 16 && !ctx->ho) {
         const int64_t sp_per_warp = own_nnz / std::max<int64_t>(1, (int64_t)ctx->sp_grid * ctx->sp_wpb);
         int64_t sp_hub_deg = std::max<int64_t>(2 * kSpHubSeg, sp_per_warp / 8);
         if (const char *ev = std::getenv("BIGCLAM_SPARSE_HUB_DEG")) sp_hub_deg = std::max<int64_t>(1, std::atoll(ev));
@@ -327,8 +337,8 @@ static int rebuild_sparse_lists(bigclam_ctx *ctx, const std::vector<NodeMeta> &m
         CU(cudaMemset(ctx->d_hub_counters, 0, sizeof(unsigned int) * (2 * (size_t)std::max<int32_t>(1, nh) + 1)));
     }
     // after the hubs: nodes above the tile budget go one per warp (general path), the rest in tiles of up to
-    // kTlMaxNodes consecutive nodes with at most tile_edges edges
-    const int32_t budget = (ctx->nsteps <= 16) ? ctx->tile_edges : 0;
+    // kTlMaxNodes consecutive nodes with at most tile_edges edges (held-out pairs: no tiles)
+    const int32_t budget = (ctx->nsteps <= 16 && !ctx->ho) ? ctx->tile_edges : 0;
     int64_t pos = nh;
     while (pos < cnt && (budget <= 0 || meta[(size_t)pos].deg > budget)) ++pos;
     ctx->n_gen = (int32_t)(pos - nh);
@@ -1078,9 +1088,12 @@ static int timed_launch(bigclam_ctx *ctx, const StepArgs &a, bool is_step) {
         sp.pr_xlo = std::nextafterf((float)a.x_lo, 0.0f);
         sp.pr_kinv = std::nextafterf((float)(1.0 / (1.0 - ctx->p.max_p)), INFINITY) * 1.000001f;
         sp.pr_cap = std::nextafterf((float)(a.t_hi - a.t_lo), INFINITY) * 1.000001f;
+        sp.ho_rowptr = ctx->d_ho_rowptr;
+        sp.ho_col = ctx->d_ho_col;
         const bool hub = a.n_hub_items > 0, push = sp.n_peers > 0;
         const int threads = 32 * ctx->sp_wpb;
-        if (hub && push) tile_step_kernel<true, true><<<ctx->sp_grid, threads, ctx->sp_smem, ctx->stream>>>(a, sp);
+        if (ctx->ho) tile_step_kernel<false, false, true><<<ctx->sp_grid, threads, ctx->sp_smem, ctx->stream>>>(a, sp);   // (no hubs, no peers)
+        else if (hub && push) tile_step_kernel<true, true><<<ctx->sp_grid, threads, ctx->sp_smem, ctx->stream>>>(a, sp);
         else if (hub) tile_step_kernel<false, true><<<ctx->sp_grid, threads, ctx->sp_smem, ctx->stream>>>(a, sp);
         else if (push) tile_step_kernel<true, false><<<ctx->sp_grid, threads, ctx->sp_smem, ctx->stream>>>(a, sp);
         else tile_step_kernel<false, false><<<ctx->sp_grid, threads, ctx->sp_smem, ctx->stream>>>(a, sp);
@@ -1402,10 +1415,128 @@ extern "C" int bigclam_get_tile_stats(bigclam_ctx *ctx, int64_t *tiles_done, int
 }
 
 // ------------------------------------------------------------------------------------------------
+// Held-out pairs (thesis p.20; DESIGN.md (f) f-5): the masked objective drops every held-out pair (u, v) from the edge
+// and the non-edge term, which leaves one linear term x_uv per pair in the per-node form (see SpGen::node).
+extern "C" int bigclam_set_holdout(bigclam_ctx *ctx, const int64_t *ho_rowptr, const int32_t *ho_col, const uint8_t *ho_is_edge) {
+    if (ctx == nullptr) return BIGCLAM_EINVAL;
+    if (!ctx->sparse) return fail(ctx, BIGCLAM_EUNSUPPORTED, "bigclam_set_holdout: needs a BIGCLAM_F_SPARSE_ROWS context");
+    if (ctx->n_peers > 0 || ctx->x_world > 0)
+        return fail(ctx, BIGCLAM_EUNSUPPORTED, "bigclam_set_holdout: the context has peers open (the masked objective runs on one GPU)");
+    const int64_t n = ctx->n;
+    bool all_owned = ctx->lo == 0 && ctx->hi == n && (int64_t)ctx->h_owned.size() == n;
+    if (all_owned) {
+        std::vector<uint8_t> seen((size_t)n, 0);
+        for (int32_t u : ctx->h_owned) {
+            if (seen[(size_t)u]) { all_owned = false; break; }
+            seen[(size_t)u] = 1;
+        }
+    }
+    if (!all_owned) return fail(ctx, BIGCLAM_EUNSUPPORTED, "bigclam_set_holdout: the context owns a node range or set (the masked objective needs all nodes)");
+    CU(cudaSetDevice(ctx->device));
+    if (ho_rowptr != nullptr) {
+        // every check before anything on the device changes
+        if (ho_rowptr[0] != 0) return fail(ctx, BIGCLAM_EINVAL, "bigclam_set_holdout: ho_rowptr[0] != 0");
+        for (int64_t u = 0; u < n; ++u)
+            if (ho_rowptr[u + 1] < ho_rowptr[u]) return fail(ctx, BIGCLAM_EINVAL, "bigclam_set_holdout: ho_rowptr not monotone at %lld", (long long)u);
+        const int64_t m = ho_rowptr[n];
+        if (m > 0 && (ho_col == nullptr || ho_is_edge == nullptr)) return fail(ctx, BIGCLAM_EINVAL, "bigclam_set_holdout: ho_col / ho_is_edge is NULL");
+        for (int64_t e = 0; e < m; ++e) {
+            if (ho_col[e] < 0 || ho_col[e] >= n) return fail(ctx, BIGCLAM_EINVAL, "bigclam_set_holdout: ho_col[%lld] out of range", (long long)e);
+            if (ho_is_edge[e] > 1) return fail(ctx, BIGCLAM_EINVAL, "bigclam_set_holdout: ho_is_edge[%lld] is neither 0 nor 1", (long long)e);
+        }
+        // per row: (partner, label) sorted by partner, and the training neighbours sorted
+        std::vector<std::pair<int32_t, uint8_t>> hs((size_t)m);
+        for (int64_t e = 0; e < m; ++e) hs[(size_t)e] = {ho_col[e], ho_is_edge[e]};
+        std::vector<int32_t> tr(ctx->h_col);
+        const std::vector<int64_t> &rp = ctx->h_rowptr;
+        for (int64_t u = 0; u < n; ++u) {
+            std::sort(hs.begin() + ho_rowptr[u], hs.begin() + ho_rowptr[u + 1]);
+            std::sort(tr.begin() + rp[u], tr.begin() + rp[u + 1]);
+        }
+        for (int64_t u = 0; u < n; ++u) {
+            for (int64_t e = ho_rowptr[u]; e < ho_rowptr[u + 1]; ++e) {
+                const int32_t v = hs[(size_t)e].first;
+                const uint8_t lab = hs[(size_t)e].second;
+                if (v == u) return fail(ctx, BIGCLAM_EINVAL, "bigclam_set_holdout: self pair at node %lld", (long long)u);
+                if (e > ho_rowptr[u] && hs[(size_t)e - 1].first == v)
+                    return fail(ctx, BIGCLAM_EINVAL, "bigclam_set_holdout: pair (%lld, %d) listed twice", (long long)u, v);
+                if (std::binary_search(tr.begin() + rp[u], tr.begin() + rp[u + 1], v))
+                    return fail(ctx, BIGCLAM_EINVAL, "bigclam_set_holdout: pair (%lld, %d) is also a training edge", (long long)u, v);
+                const auto vb = hs.begin() + ho_rowptr[v], ve = hs.begin() + ho_rowptr[v + 1];
+                const auto it = std::lower_bound(vb, ve, std::make_pair((int32_t)u, (uint8_t)0));
+                if (it == ve || it->first != (int32_t)u)
+                    return fail(ctx, BIGCLAM_EINVAL, "bigclam_set_holdout: pair (%lld, %d) has no mirror (%d, %lld)", (long long)u, v, v, (long long)u);
+                if (it->second != lab)
+                    return fail(ctx, BIGCLAM_EINVAL, "bigclam_set_holdout: pair (%lld, %d) and its mirror have different labels", (long long)u, v);
+            }
+        }
+        if (int rd = drop_speculation(ctx)) return rd;
+        CU(cudaStreamSynchronize(ctx->stream));
+        cudaFree(ctx->d_ho_rowptr); cudaFree(ctx->d_ho_col); cudaFree(ctx->d_ho_edge); cudaFree(ctx->d_ho_part);
+        ctx->d_ho_rowptr = nullptr; ctx->d_ho_col = nullptr; ctx->d_ho_edge = nullptr; ctx->d_ho_part = nullptr;
+        ctx->ho = false;
+        CU(cudaMalloc(&ctx->d_ho_rowptr, sizeof(int64_t) * ((size_t)n + 1)));
+        CU(cudaMalloc(&ctx->d_ho_col, sizeof(int32_t) * std::max<size_t>(1, (size_t)m)));
+        CU(cudaMalloc(&ctx->d_ho_edge, std::max<size_t>(1, (size_t)m)));
+        CU(cudaMalloc(&ctx->d_ho_part, sizeof(double) * ((size_t)n + 1)));
+        CU(cudaMemcpy(ctx->d_ho_rowptr, ho_rowptr, sizeof(int64_t) * ((size_t)n + 1), cudaMemcpyHostToDevice));
+        if (m > 0) {
+            CU(cudaMemcpy(ctx->d_ho_col, ho_col, sizeof(int32_t) * (size_t)m, cudaMemcpyHostToDevice));
+            CU(cudaMemcpy(ctx->d_ho_edge, ho_is_edge, (size_t)m, cudaMemcpyHostToDevice));
+        }
+        CU(cudaFuncSetAttribute(tile_step_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->sp_smem));
+        CU(cudaFuncSetAttribute(holdout_llh_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(double) * kHoWarps * (size_t)sp_ldp(ctx->ld))));
+        ctx->ho_pairs = m / 2;
+        ctx->ho = true;
+    } else {
+        if (int rd = drop_speculation(ctx)) return rd;
+        CU(cudaStreamSynchronize(ctx->stream));
+        cudaFree(ctx->d_ho_rowptr); cudaFree(ctx->d_ho_col); cudaFree(ctx->d_ho_edge); cudaFree(ctx->d_ho_part);
+        ctx->d_ho_rowptr = nullptr; ctx->d_ho_col = nullptr; ctx->d_ho_edge = nullptr; ctx->d_ho_part = nullptr;
+        ctx->ho_pairs = 0;
+        ctx->ho = false;
+    }
+    std::vector<int32_t> order = ctx->h_owned;            // the routing follows ctx->ho (rebuild_sparse_lists)
+    return rebuild_order_list(ctx, ctx->h_rowptr, order);
+}
+
+extern "C" int bigclam_holdout_loglikelihood(bigclam_ctx *ctx, double *llh_out, int64_t *n_pairs_out) {
+    if (ctx == nullptr) return BIGCLAM_EINVAL;
+    if (llh_out == nullptr) return fail(ctx, BIGCLAM_EINVAL, "bigclam_holdout_loglikelihood: llh_out is NULL");
+    if (!ctx->ho) return fail(ctx, BIGCLAM_EINVAL, "bigclam_holdout_loglikelihood: no held-out pairs (bigclam_set_holdout)");
+    CU(cudaSetDevice(ctx->device));
+    const bigclam_params &p = ctx->p;
+    HoLlhArgs h{};
+    h.hdr = ctx->d_hdr[ctx->cur];
+    h.pool = ctx->d_pool[ctx->cur];
+    h.ho_rowptr = ctx->d_ho_rowptr;
+    h.ho_col = ctx->d_ho_col;
+    h.ho_edge = ctx->d_ho_edge;
+    h.n = ctx->n;
+    h.ld = ctx->ld;
+    h.min_p = p.min_p;
+    h.max_p = p.max_p;
+    h.x_lo = -std::log(p.max_p) * (1.0 - 1e-12);           // (fill_args)
+    h.x_hi = -std::log(p.min_p) * (1.0 + 1e-12);
+    h.part = ctx->d_ho_part;
+    const unsigned blocks = (unsigned)((ctx->n + kHoWarps - 1) / kHoWarps);
+    holdout_llh_kernel<<<blocks, kHoWarps * 32, sizeof(double) * kHoWarps * (size_t)sp_ldp(ctx->ld), ctx->stream>>>(h);
+    CU(cudaGetLastError());
+    holdout_sum_kernel<<<1, kHoSumThreads, 0, ctx->stream>>>(ctx->d_ho_part, ctx->n, ctx->d_ho_part + ctx->n);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(ctx->h_pinned, ctx->d_ho_part + ctx->n, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    *llh_out = ctx->h_pinned[0];
+    if (n_pairs_out) *n_pairs_out = ctx->ho_pairs;
+    return BIGCLAM_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
 // Node-partitioned pieces (DESIGN.md (e)).
 extern "C" int bigclam_set_owned_range(bigclam_ctx *ctx, int64_t lo, int64_t hi) {
     if (ctx == nullptr) return BIGCLAM_EINVAL;
     if (lo < 0 || hi < lo || hi > ctx->n) return fail(ctx, BIGCLAM_EINVAL, "bigclam_set_owned_range: bad range");
+    if (ctx->ho) return fail(ctx, BIGCLAM_EUNSUPPORTED, "bigclam_set_owned_range: the context has held-out pairs (bigclam_set_holdout)");
     CU(cudaSetDevice(ctx->device));
     const std::vector<int64_t> &rp = ctx->h_rowptr;
     ctx->lo = lo;
@@ -1514,6 +1645,7 @@ extern "C" int bigclam_ipc_export(bigclam_ctx *ctx, void *handles_out /* 2 x 64 
 extern "C" int bigclam_ipc_open_peers(bigclam_ctx *ctx, int32_t world, int32_t rank, const void *all_handles /* world x 2 x 64 */) {
     if (ctx == nullptr || all_handles == nullptr || world < 1 || world > 8 || rank < 0 || rank >= world)
         return fail(ctx, BIGCLAM_EINVAL, "bigclam_ipc_open_peers: bad world/rank (at most 8 GPUs)");
+    if (ctx->ho) return fail(ctx, BIGCLAM_EUNSUPPORTED, "bigclam_ipc_open_peers: the context has held-out pairs (bigclam_set_holdout)");
     CU(cudaSetDevice(ctx->device));
     const cudaIpcMemHandle_t *h = reinterpret_cast<const cudaIpcMemHandle_t *>(all_handles);
     for (int half = 0; half < 2; ++half)            // a second call replaces the first mapping
@@ -1598,6 +1730,7 @@ extern "C" int bigclam_set_owned_nodes(bigclam_ctx *ctx, const int32_t *nodes, i
     if (ctx == nullptr) return BIGCLAM_EINVAL;
     if (count < 0 || count > ctx->n || (count > 0 && nodes == nullptr))
         return fail(ctx, BIGCLAM_EINVAL, "bigclam_set_owned_nodes: bad node list");
+    if (ctx->ho) return fail(ctx, BIGCLAM_EUNSUPPORTED, "bigclam_set_owned_nodes: the context has held-out pairs (bigclam_set_holdout)");
     for (int64_t i = 0; i < count; ++i)
         if (nodes[i] < 0 || nodes[i] >= ctx->n) return fail(ctx, BIGCLAM_EINVAL, "bigclam_set_owned_nodes: node out of range");
     CU(cudaSetDevice(ctx->device));
@@ -1639,6 +1772,7 @@ extern "C" int bigclam_extract(bigclam_ctx *ctx, double delta, uint8_t *member_o
 static int xchg_alloc(bigclam_ctx *ctx, int32_t world, int32_t rank) {
     if (world < 1 || world > 8 || rank < 0 || rank >= world) return fail(ctx, BIGCLAM_EINVAL, "exchange buffers: bad world/rank (at most 8 GPUs)");
     if (!ctx->sparse) return fail(ctx, BIGCLAM_EUNSUPPORTED, "the fused collective needs BIGCLAM_F_SPARSE_ROWS");
+    if (ctx->ho) return fail(ctx, BIGCLAM_EUNSUPPORTED, "exchange buffers: the context has held-out pairs (bigclam_set_holdout)");
     CU(cudaSetDevice(ctx->device));
     cudaFree(ctx->d_xbuf); ctx->d_xbuf = nullptr;
     cudaFree(ctx->d_xflags); ctx->d_xflags = nullptr;
@@ -1669,6 +1803,7 @@ extern "C" int bigclam_xchg_export(bigclam_ctx *ctx, int32_t world, int32_t rank
 extern "C" int bigclam_xchg_open_peers(bigclam_ctx *ctx, const void *all_handles /* world x 2 x 64 bytes, rank order */) {
     if (ctx == nullptr || all_handles == nullptr) return BIGCLAM_EINVAL;
     if (ctx->x_world < 1) return fail(ctx, BIGCLAM_EINVAL, "bigclam_xchg_open_peers: call bigclam_xchg_export first");
+    if (ctx->ho) return fail(ctx, BIGCLAM_EUNSUPPORTED, "bigclam_xchg_open_peers: the context has held-out pairs (bigclam_set_holdout)");
     CU(cudaSetDevice(ctx->device));
     const cudaIpcMemHandle_t *h = reinterpret_cast<const cudaIpcMemHandle_t *>(all_handles);
     for (int r = 0; r < ctx->x_world; ++r) {

@@ -102,6 +102,10 @@ struct SparseArgs {
     // 1 = bounds on the tile path only, 2 = on the general path too
     int32_t ls_prune;
     float pr_xlo, pr_kinv, pr_cap;     // x_lo rounded down, 1 / (1 - MAX_P_) and S_hi - S_lo rounded up
+    // held-out pairs (bigclam_set_holdout): node u's partners ho_col[ho_rowptr[u] .. ho_rowptr[u + 1]); read only by the
+    // masked (kHO) instantiation of the step kernel
+    const int64_t *ho_rowptr;
+    const int32_t *ho_col;
 };
 
 // The dense per-warp vectors are padded to a multiple of 32 components (zeros: a padding component has
@@ -258,7 +262,9 @@ struct SpGen {
     }
 
     // PRE over the edges [eb, ee) of a node whose fu is in fu_d: returns this lane's share of S1 (lane e holds the
-    // terms of the chunks' e-th rows); with `axpy` the weighted neighbour rows are added into g_d.
+    // terms of the chunks' e-th rows); with `axpy` the weighted neighbour rows are added into g_d.  kLin: the pairs are
+    // held-out pairs, whose term in the masked objective is x itself with weight 1.
+    template <bool kLin = false>
     __device__ __forceinline__ double pre_range(const int32_t *colbase, int eb, int ee, bool axpy, int &nchunks, int &ne_last) {
         double S1 = 0.0;
         nchunks = 0;
@@ -272,8 +278,13 @@ struct SpGen {
 #pragma unroll 1
                 for (int i = poff[lane]; i < end; ++i) x = fma(ent_val[i], fu_d[ent_idx[i]], x);
             }
-            double w;
-            const double t = edge_term<true>(x, ec, w);
+            double w, t;
+            if constexpr (kLin) {
+                t = x;
+                w = 1.0;
+            } else {
+                t = edge_term<true>(x, ec, w);
+            }
             S1 += (lane < ne) ? t : 0.0;
             if (axpy) {
 #pragma unroll 1
@@ -355,7 +366,9 @@ struct SpGen {
         __syncwarp();
     }
     // Line search over the edges [eb, ee): lane (j, h) returns the sum over its edges of the clamped edge term
-    // for candidate step s; `staged` rows of a single chunk may still be in the buffer from PRE.
+    // for candidate step s; `staged` rows of a single chunk may still be in the buffer from PRE.  kLin: held-out
+    // pairs, the term is the dot nf_j.fv itself.
+    template <bool kLin = false>
     __device__ __forceinline__ double ls_range(const int32_t *colbase, int eb, int ee, double s, bool need_hi, int staged) {
         const int h = lane >> 4;
         const double max_f = a->max_f;
@@ -387,7 +400,12 @@ struct SpGen {
                     }
                 }
                 double tA, tB;
-                edge_term2(DA, DB, ec, tA, tB);
+                if constexpr (kLin) {
+                    tA = DA;
+                    tB = DB;
+                } else {
+                    edge_term2(DA, DB, ec, tA, tB);
+                }
                 sumterms += vA ? tA : 0.0;
                 sumterms += vB ? tB : 0.0;
             }
@@ -625,7 +643,10 @@ struct SpGen {
     }
 
     // One node, start to finish.  colp: the node's neighbour list (ids in the low 28 bits when it comes from tcol).
-    template <bool kPush>
+    // kHO (masked objective, bigclam_set_holdout): the node's held-out list is walked after its neighbour list, each
+    // pair with the linear term x_uv (PRE: S1 += x, g += fv; line search: sumterms += nf_j.fv); the bounds stay off,
+    // they were derived for the unmasked objective.
+    template <bool kPush, bool kHO = false>
     __device__ BIGCLAM_GEN_INLINE void node(int64_t u, int deg, const int32_t *colp) {
         const uint64_t hu = __ldg(sp->hdr_in + u);
         const int cu = (int)sp_cnt(hu);
@@ -640,7 +661,17 @@ struct SpGen {
 
         // ---------------- PRE (:157-169) ----------------
         int nchunks, ne_last;
-        const double S1 = warp_sum(pre_range(colp, 0, deg, want_ls, nchunks, ne_last));
+        double S1 = pre_range(colp, 0, deg, want_ls, nchunks, ne_last);
+        int hdeg = 0;                                   // held-out pairs of the node (kHO)
+        const int32_t *hcol = nullptr;
+        if constexpr (kHO) {
+            const int64_t h0 = __ldg(sp->ho_rowptr + u);
+            hdeg = (int)(__ldg(sp->ho_rowptr + u + 1) - h0);
+            hcol = sp->ho_col + h0;
+            int hch, hnl;
+            S1 += pre_range<true>(hcol, 0, hdeg, want_ls, hch, hnl);
+        }
+        S1 = warp_sum(S1);
         const double llh_u = (S1 - fusf) + fufu;
         int jstar = -1, m = 0;
         if (want_ls) {
@@ -648,7 +679,7 @@ struct SpGen {
             const double G2 = scan_gradient(m, need_hi);
             // ---------------- LS (:172-182): only if the bounds leave a candidate that can pass ----------------
             unsigned surv = 0xffffu;
-            if (BIGCLAM_GEN_BOUNDS && sp->ls_prune > 1 && nsteps <= 16) surv = bound_mask(colp, deg, m, G2, llh_u, fusf, fufu, nchunks == 1 ? ne_last : 0);
+            if (!kHO && BIGCLAM_GEN_BOUNDS && sp->ls_prune > 1 && nsteps <= 16) surv = bound_mask(colp, deg, m, G2, llh_u, fusf, fufu, nchunks == 1 ? ne_last : 0);
             if (sp->stats != nullptr && lane == 0) {
                 atomicAdd(sp->stats + 3, 1u);
                 if (surv != 0u) atomicAdd(sp->stats + 2, 1u);
@@ -658,8 +689,10 @@ struct SpGen {
                 const int j = tg + j16;
                 const bool jok = j < nsteps;
                 const double s = s_steps[jok ? j : 0];
-                // a node whose neighbours fitted one chunk still has them staged from PRE
-                double sumterms = ls_range(colp, 0, deg, s, need_hi, (nchunks == 1 && tg == 0) ? ne_last : 0);
+                // a node whose neighbours fitted one chunk still has them staged from PRE (unless held-out pairs
+                // were staged after them)
+                double sumterms = ls_range(colp, 0, deg, s, need_hi, (nchunks == 1 && tg == 0 && hdeg == 0) ? ne_last : 0);
+                if constexpr (kHO) sumterms += ls_range<true>(hcol, 0, hdeg, s, need_hi, 0);
                 sumterms += __shfl_xor_sync(0xffffffffu, sumterms, 16);
                 jstar = decide(tg, s, jok, sumterms, m, need_hi, llh_u, G2, surv);
             }
@@ -790,6 +823,82 @@ struct SpGen {
         __syncwarp();
     }
 };
+
+// ---------------------------------------------------------------------------------------------------------------
+// Held-out log-likelihood of the current F (bigclam_holdout_loglikelihood), every held-out pair once (u < v):
+//   L_HO = sum over held-out edges of log(1 - p) + sum over held-out non-edges of log(p),  p = clamp(exp(-Fu.Fv)) (:166).
+// One warp per node u scatters u's row into its dense shared-memory vector; lane l scores the pairs (u, v), v > u, at
+// positions l, l + 32, ... of u's list by gathering v's entries as PRE does.  Per-node partials (each lane's terms in
+// list order, then a fixed butterfly) go to part[u]; holdout_sum_kernel adds them up in node order: reruns give the
+// same bits.  The list is here sorted-or-not, symmetric and free of self pairs (bigclam_set_holdout checks).
+struct HoLlhArgs {
+    const uint64_t *hdr;
+    const double *pool;
+    const int64_t *ho_rowptr;
+    const int32_t *ho_col;
+    const uint8_t *ho_edge;
+    int64_t n;
+    int32_t ld;
+    double min_p, max_p;
+    double x_lo, x_hi;        // as StepArgs: exp(-x) is only evaluated in between, the clamp decides outside
+    double *part;             // n
+};
+constexpr int kHoWarps = 8;
+
+__global__ void __launch_bounds__(kHoWarps * 32) holdout_llh_kernel(const HoLlhArgs h) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    const int64_t u = (int64_t)blockIdx.x * kHoWarps + wib;
+    if (u >= h.n) return;                                   // (warp-uniform)
+    const int ldp = sp_ldp(h.ld);
+    double *fu_d = reinterpret_cast<double *>(smem_raw) + (size_t)wib * ldp;
+    const int64_t b = h.ho_rowptr[u], e = h.ho_rowptr[u + 1];
+    double acc = 0.0;
+    if (e > b) {
+        for (int i = lane; i < ldp; i += 32) fu_d[i] = 0.0;
+        __syncwarp();
+        const uint64_t hu = h.hdr[u];
+        const int cu = (int)sp_cnt(hu);
+        const double *uval = h.pool + sp_off8(hu);
+        const unsigned short *uidx = sp_idx(uval, (uint32_t)cu);
+        for (int i = lane; i < cu; i += 32) fu_d[uidx[i]] = uval[i];
+        __syncwarp();
+        for (int64_t q = b + lane; q < e; q += 32) {
+            const int v = h.ho_col[q];
+            if (v <= u) continue;
+            const uint64_t hv = __ldg(h.hdr + v);
+            const int cv = (int)sp_cnt(hv);
+            const double *vval = h.pool + sp_off8(hv);
+            const unsigned short *vidx = sp_idx(vval, (uint32_t)cv);
+            double x = 0.0;
+            for (int i = 0; i < cv; ++i) x = fma(__ldg(vval + i), fu_d[__ldg(vidx + i)], x);
+            const bool inside = (x > h.x_lo) && (x < h.x_hi);
+            double p = inside ? exp_neg(x) : (x <= h.x_lo ? h.max_p : h.min_p);
+            p = fmin(fmax(p, h.min_p), h.max_p);
+            acc += log_pos(h.ho_edge[q] ? 1.0 - p : p);
+        }
+    }
+    acc = warp_sum(acc);
+    if (lane == 0) h.part[u] = acc;
+}
+
+// sum_u part[u] in a fixed order: thread t adds a contiguous range front to back, the threads' sums meet in a fixed tree.
+constexpr int kHoSumThreads = 256;
+__global__ void __launch_bounds__(kHoSumThreads) holdout_sum_kernel(const double *part, int64_t n, double *out) {
+    __shared__ double s_sum[kHoSumThreads];
+    const int t = threadIdx.x;
+    const int64_t per = (n + kHoSumThreads - 1) / kHoSumThreads;
+    const int64_t b = (int64_t)t * per, e = (b + per < n) ? b + per : n;
+    double v = 0.0;
+    for (int64_t i = b; i < e; ++i) v += part[i];
+    s_sum[t] = v;
+    __syncthreads();
+    for (int o = kHoSumThreads / 2; o > 0; o >>= 1) {
+        if (t < o) s_sum[t] += s_sum[t + o];
+        __syncthreads();
+    }
+    if (t == 0) *out = s_sum[0];
+}
 
 // Dense n x ld rows -> sparse rows (one warp per row; non-zeros in ascending component order).
 __global__ void dense_to_sparse_kernel(const double *F, int64_t n, int ld, uint64_t *hdr, double *pool,

@@ -1027,8 +1027,9 @@ BIGCLAM_UNROLL(BIGCLAM_TL_UJ)
 };
 
 // kPush: multi-GPU launch, the peers' replicas are written too; kHub: the launch has split hubs.  Both are
-// compile-time so that the plain single-GPU kernel carries none of that code.
-template <bool kPush, bool kHub>
+// compile-time so that the plain single-GPU kernel carries none of that code.  kHO: the masked objective of a context
+// with held-out pairs (bigclam_set_holdout): every node goes through the general path (no tiles, no split hubs).
+template <bool kPush, bool kHub, bool kHO = false>
 __global__ void __launch_bounds__(kTlThreads, kTlBlocksPerSM) tile_step_kernel(const __grid_constant__ StepArgs a, const __grid_constant__ SparseArgs sp) {
     if (a.done_flag != nullptr && *a.done_flag != 0) return;
 
@@ -1091,7 +1092,7 @@ __global__ void __launch_bounds__(kTlThreads, kTlBlocksPerSM) tile_step_kernel(c
         }
     }
 
-    const unsigned int n_items = (unsigned int)sp.n_gen + (unsigned int)sp.ntiles;
+    const unsigned int n_items = (unsigned int)sp.n_gen + (kHO ? 0u : (unsigned int)sp.ntiles);
     unsigned int item = 0;
     if (lane == 0) item = atomicAdd(a.work_counter, 1u);
     item = __shfl_sync(0xffffffffu, item, 0);
@@ -1102,7 +1103,7 @@ __global__ void __launch_bounds__(kTlThreads, kTlBlocksPerSM) tile_step_kernel(c
         int gen_cnt = 1;
         int64_t gen_pos = (int64_t)a.n_hubs + item;
         const int32_t *gen_col = nullptr;
-        if (item >= (unsigned int)sp.n_gen) {
+        if (!kHO && item >= (unsigned int)sp.n_gen) {
             const TileMeta tm = sp.tiles[item - (unsigned int)sp.n_gen];
             dense_clean = false;
             const bool done = T.template run<kPush>(tm);
@@ -1118,7 +1119,7 @@ __global__ void __launch_bounds__(kTlThreads, kTlBlocksPerSM) tile_step_kernel(c
         for (int i = 0; i < gen_cnt; ++i) {
             const NodeMeta nm = a.meta[gen_pos + i];
             if (!dense_clean) { G.clear_dense(); dense_clean = true; }
-            G.template node<kPush>(nm.u, nm.deg, gen_col != nullptr ? gen_col : a.col + nm.e0);
+            G.template node<kPush, kHO>(nm.u, nm.deg, gen_col != nullptr ? gen_col : a.col + nm.e0);
             if (gen_col != nullptr) gen_col += nm.deg;
         }
         item = __shfl_sync(0xffffffffu, nxt, 0);

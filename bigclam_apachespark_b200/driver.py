@@ -358,6 +358,85 @@ class BigClam:
             LLHKold = LLHKnew
         return KforC, hist
 
+    # ---- K by held-out likelihood (the thesis p.20; holdout.py, DESIGN.md (f) f-5) ----
+    def set_holdout(self, ho_rowptr, ho_col, ho_is_edge):
+        """Held-out pairs of the current context (sparse rows, one GPU): from now on the steps, SGDFindC and
+        loglikelihood() use the masked objective, which leaves every held-out pair out.  Symmetric lists, disjoint from
+        the neighbour lists; ho_is_edge = 1 for a held-out edge, 0 for a held-out non-edge (holdout.split_pairs makes
+        them).  The lists belong to the context: set_K() or a new graph drops them."""
+        if self._multi is not None:
+            raise RuntimeError("held-out pairs are single-GPU only (numGPUs = 1)")
+        rp = np.ascontiguousarray(ho_rowptr, dtype=np.int64)
+        hc = np.ascontiguousarray(ho_col, dtype=np.int32)
+        he = np.ascontiguousarray(ho_is_edge, dtype=np.uint8)
+        if len(rp) != self.n + 1 or len(hc) != rp[-1] or len(he) != rp[-1]:
+            raise ValueError("held-out CSR arrays do not describe n rows")
+        check(_lib.load().bigclam_set_holdout(self._need(), rp.ctypes.data, hc.ctypes.data, he.ctypes.data), self._ctx)
+        return self
+
+    def clear_holdout(self):
+        """Back to the unmasked objective (exactly as if no held-out pairs had been set)."""
+        if self._ctx is not None:
+            check(_lib.load().bigclam_set_holdout(self._ctx, None, None, None), self._ctx)
+        return self
+
+    def holdout_loglikelihood(self) -> float:
+        """Log-likelihood of the held-out pairs under the current F: sum of log(1 - p) over held-out edges plus sum of
+        log(p) over held-out non-edges, p = clamp(exp(-Fu.Fv)), each pair once.  Sets last_holdout_pairs."""
+        llh = C.c_double()
+        npairs = C.c_int64()
+        check(_lib.load().bigclam_holdout_loglikelihood(self._need(), C.byref(llh), C.byref(npairs)), self._ctx)
+        self.last_holdout_pairs = npairs.value
+        return llh.value
+
+    def select_K(self, Ks=None, ho_frac: float = 0.2, repeats: int = 3, seed: int = 0, max_outer: int = 0, refit: bool = True):
+        """Chooses K by held-out likelihood.  For every K (default: Kset()) and repeat r the graph is split with seed
+        seed + r (holdout.split_pairs: ho_frac of the edges and as many non-edges); on the TRAINING graph
+        conductanceLocalMin(), initNeighborComF(K), set_holdout and SGDFindC(max_outer) run, then the held-out pairs are
+        scored.  K_best has the highest mean over the repeats (ties: the smaller K).  Returns (K_best, rows), rows =
+        [(K, mean, [value per repeat], [SGDFindC calls per repeat]), ...].  Sparse rows are used whatever the constructor
+        flags.  With refit the solver is left on the full graph at K_best, fitted by SGDFindC(max_outer) with the
+        constructor's flags and ready for communities.extract; otherwise it is left on the full graph with no context."""
+        from .holdout import split_pairs
+        if self.numGPUs > 1:
+            raise ValueError("select_K runs on one GPU (numGPUs = 1)")
+        if self.rowptr is None:
+            raise ValueError("load a graph first")
+        if repeats < 1:
+            raise ValueError("repeats must be >= 1")
+        Ks = [int(k) for k in (self.Kset() if Ks is None else Ks)]
+        full = (self.rowptr, self.col, self.ids)
+        flags = self.flags
+        splits = [split_pairs(full[0], full[1], ho_frac, seed + r) for r in range(repeats)]
+        seeds = [None] * repeats
+        rows = []
+        try:
+            self.flags = flags | _lib.F_SPARSE_ROWS
+            for K in Ks:
+                vals, calls = [], []
+                for r, sp in enumerate(splits):
+                    self.set_graph(sp.rowptr, sp.col, full[2])
+                    if seeds[r] is None:
+                        seeds[r] = self.conductanceLocalMin()
+                    self.Sbc = seeds[r]
+                    self.initNeighborComF(K)
+                    self.set_holdout(sp.ho_rowptr, sp.ho_col, sp.ho_is_edge)
+                    self.SGDFindC(max_outer=max_outer)
+                    vals.append(self.holdout_loglikelihood())
+                    calls.append(self.last_calls)
+                    if self.verbose:
+                        print(str(K) + " repeat " + str(r) + " held-out LLH: " + repr(vals[-1]))
+                rows.append((K, float(np.mean(vals)), vals, calls))
+        finally:
+            self.flags = flags
+            self.set_graph(*full)
+        K_best = max(rows, key=lambda row: (row[1], -row[0]))[0]
+        if refit:
+            self.conductanceLocalMin()
+            self.initNeighborComF(K_best)
+            self.SGDFindC(max_outer=max_outer)
+        return K_best, rows
+
     # ---- diagnostics ----
     def accepted(self) -> np.ndarray:
         out = np.empty(self.n, dtype=np.int8)

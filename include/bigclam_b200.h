@@ -138,6 +138,22 @@ int bigclam_get_tile_stats(bigclam_ctx *ctx, int64_t *tiles_done, int64_t *tiles
  * counted), how many had at least one candidate that the bounds could not exclude (and were therefore evaluated). */
 int bigclam_get_ls_stats(bigclam_ctx *ctx, int64_t *nodes_asked, int64_t *nodes_searched);
 
+/*
+ * Held-out pairs, for choosing K by held-out likelihood (BigCLAM, Yang & Leskovec; the thesis p.20).  Symmetric lists
+ * ho_rowptr[n+1] / ho_col: the held-out partners of every node; ho_is_edge[e] = 1 for a held-out edge, 0 for a held-out
+ * non-edge.  No self pairs, no pair twice in a list, no pair that is also in the context's neighbour lists.  From now
+ * on bigclam_step / bigclam_run / bigclam_loglikelihood use the masked objective: every held-out pair is left out of
+ * both the edge term and the non-edge term, i.e. llh_u gains sum_{v in HO(u)} Fu.Fv and grad_u gains sum_{v in HO(u)} Fv
+ * (DESIGN.md (f) f-5).  NULL ho_rowptr clears the lists and restores the unmasked behaviour exactly.  Sparse-rows
+ * contexts on one GPU only: BIGCLAM_EUNSUPPORTED for a dense context, one that owns a node range or set, or one with
+ * peers open; any input error is BIGCLAM_EINVAL and leaves the context as it was.
+ */
+int bigclam_set_holdout(bigclam_ctx *ctx, const int64_t *ho_rowptr, const int32_t *ho_col, const uint8_t *ho_is_edge);
+/* L_HO of the current F over every held-out pair once: sum of log(1 - p) over held-out edges plus sum of log(p) over
+ * held-out non-edges, p = clamp(exp(-Fu.Fv), min_p, max_p) (bigclam4-7.scala:166).  n_pairs_out (optional) = number
+ * of unordered pairs scored.  Same bits on every run. */
+int bigclam_holdout_loglikelihood(bigclam_ctx *ctx, double *llh_out, int64_t *n_pairs_out);
+
 /* Sparse rows: re-cut the tiles of small nodes for the current average row size (rows grow or shrink while the solver
  * runs; bigclam_run does this by itself between its batches, bigclam_set_F* always).  Synchronises the stream. */
 int bigclam_retile(bigclam_ctx *ctx);

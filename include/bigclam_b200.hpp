@@ -194,6 +194,24 @@ public:
         run(version, rel_tol, max_outer);
     }
 
+    // Held-out pairs (bigclam_set_holdout: sparse rows, one GPU): the masked objective from now on; an empty ho_rowptr
+    // clears the lists.  holdout_loglikelihood(): L_HO of the current F (n_pairs: unordered pairs scored).
+    void set_holdout(const std::vector<int64_t> &ho_rowptr, const std::vector<int32_t> &ho_col, const std::vector<uint8_t> &ho_is_edge) {
+        need();
+        if (multi_ != nullptr) throw Error(BIGCLAM_EUNSUPPORTED, "set_holdout: single-GPU contexts only");
+        if (ho_rowptr.empty()) { check(bigclam_set_holdout(ctx_, nullptr, nullptr, nullptr), "set_holdout"); return; }
+        if ((int64_t)ho_rowptr.size() != n_ + 1 || (int64_t)ho_col.size() != ho_rowptr.back() || ho_is_edge.size() != ho_col.size())
+            throw Error(BIGCLAM_EINVAL, "set_holdout: the arrays do not describe n rows");
+        check(bigclam_set_holdout(ctx_, ho_rowptr.data(), ho_col.data(), ho_is_edge.data()), "set_holdout");
+    }
+    double holdout_loglikelihood(int64_t *n_pairs = nullptr) {
+        need();
+        if (multi_ != nullptr) throw Error(BIGCLAM_EUNSUPPORTED, "holdout_loglikelihood: single-GPU contexts only");
+        double llh = 0.0;
+        check(bigclam_holdout_loglikelihood(ctx_, &llh, n_pairs), "holdout_loglikelihood");
+        return llh;
+    }
+
     // Community extraction as coded in Bigclamv2.scala:223-230.  delta_threshold: `e = 2.0*count/(N*(N-1)); sqrt(-log(1-e))`
     // (:223-224; in the script `count` is the number of vertices that have edges, the thesis uses |E|: pass what you mean).
     // extract(): communities[c] = vertices u with F_uc >= delta, or, when the row maximum is below delta, with F_uc equal to
